@@ -29,6 +29,11 @@ One JSON line is printed by rank 0.  `value` = whole-job Msamples/s with the IQ 
 timed region); `roofline` = the demod kernel against the measured HBM copy bandwidth;
 `cpu_baseline` = the CPU restatement timed on this box (bounded sample); `sustained` = the same
 step repeated for >= 2 s.
+
+`--dump-outputs DIR` (GPU arm) writes, for each workload, what the last of the K timed steps
+returned: the candidate records of ertgpu_fetch and the counters of ertgpu_last_counts, as
+float64 / float32 arrays DIR/<workload>_<field>.npy (see dump_outputs).  The inputs are seeded,
+so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -73,7 +78,12 @@ def parse_args():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-threads", type=int, default=0, help="reference arm: threads (default: every CPU the process may use)")
     ap.add_argument("--no-numa-bind", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step of each workload returned as DIR/<workload>_<field>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_config(name, w, nbytes_per_gpu, world, bs, pkl):
@@ -256,6 +266,8 @@ def cpu_rate(msgtype, iq, nthreads: int, repeats: int = 1):
 
 
 def run_reference(args):
+    if args.dump_outputs:
+        raise SystemExit("--dump-outputs: the reference arm returns counts only; dumps come from the GPU arm")
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return 0
@@ -421,6 +433,9 @@ def measure(job, args, barrier, sampler, stream, with_e2e, sustained_s):
     ms_total, launches, t_wall0, t_wall1 = timed(args.steps)
     out = {"ms_total": ms_total, "launches": launches, "n_pkts": n_pkts,
            "clocks": sampler.window(t_wall0, t_wall1) if sampler else None}
+    if args.dump_outputs:
+        # the last timed step's results are still in the handle: read them back outside the timed window
+        out["records"], out["counts"] = h.fetch(1 << 20), h.last_counts()
     # timed region 2: the same K steps with CUDA events recorded by the library around each stage (the roofline's
     # kernel time); the events sit between the kernels, so this pass runs them strictly one after another
     h.set_stage_timing(True)
@@ -547,6 +562,32 @@ def summarise(job, args, raw, world, peak, peak_src):
     return res
 
 
+DUMP_BYTES = 60 << 20   # --dump-outputs: the rows of all workloads together; with the .npy headers under 64 MB
+
+
+def dump_outputs(directory, tag, job, records, counts, budget):
+    """DIR/<tag>_<field>.npy: the candidate records a caller gets from ertgpu_fetch, in (block, preamble_id, idx)
+    order, one array per field -- block, idx, preamble_id, check_mask, flags (float64), bytes[:, :packet_bytes]
+    and, for r900 workloads, r900_digits (float32) -- plus `counts` = ertgpu_last_counts (candidates, valid).
+    If the records need more than `budget` bytes, a fixed seeded sample of rows is kept; `row` holds the
+    record numbers written either way."""
+    import numpy as np
+    cols = {f: records[f].astype(np.float64) for f in ("block", "idx", "preamble_id", "check_mask", "flags")}
+    cols["bytes"] = records["bytes"][:, :job.cfg.packet_bytes].astype(np.float32)
+    if any(m.startswith("r900") for m in job.msgtypes):
+        cols["r900_digits"] = records["r900_digits"].astype(np.float32)
+    row_bytes = 8 + sum(c.itemsize * (c.size // max(1, len(c))) for c in cols.values())
+    rows = np.arange(len(records))
+    if len(rows) * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(len(rows), budget // row_bytes, replace=False))
+    cols = {k: v[rows] for k, v in cols.items()}
+    cols["row"] = rows.astype(np.float64)
+    cols["counts"] = np.array(counts, dtype=np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for k, v in cols.items():
+        np.save(os.path.join(directory, f"{tag}_{k}.npy"), v)
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -597,6 +638,9 @@ def run_b200(args):
         job = Job(name, args, world, rank, local)
         head = i == 0
         raw = measure(job, args, barrier, sampler, stream, with_e2e=head, sustained_s=args.sustained_seconds if head else 0.0)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, name if world == 1 else f"{name}_rank{rank}", job, raw["records"], raw["counts"],
+                         DUMP_BYTES // (len(names) * world))
         mx = [raw["ms_total"], raw.get("e2e_s", 0.0), raw.get("e2e_pageable_s", 0.0), raw["sustained"]["ms_total"] if "sustained" in raw else 0.0]
         sm = [float(raw["n_pkts"])]
         mx, sm = reduce_over_ranks(world, mx, sm)
